@@ -115,6 +115,32 @@ def geometry_bytes(cfg, nlevels=8, scale=1.2):
     return {"k_warp": Iw * Ih + 5 * W * W, "k_pyramid": sum(sizes[:-1]) + sum(sizes[1:]), "k_fast": sum(sizes), "levels_px": sizes, "fast_scored_px": scored}
 
 
+DUMP_FRAMES = 32     # frames whose full results --dump-outputs writes (a fixed, seeded sample; counts are written for every frame)
+
+
+def dump_outputs(out_dir, kps, desc, nout, match, nmatch):
+    """What the last timed step returned to its caller, as .npy files for comparing two builds output for output: per frame the key point
+    and match counts, and for a seeded sample of frames the key points (x, y, size, angle, response, octave, class_id), the 32 descriptor
+    bytes and the match index of every key point in the next frame. Entries past a frame's count (and the match row of the last frame,
+    which has no next frame) are not computed by the step and are written as 0 / -1."""
+    frames, cap = kps.shape[0], kps.shape[1]
+    n = nout.cpu().numpy().astype(np.int64)
+    pick = np.sort(np.random.default_rng(0).choice(frames, min(DUMP_FRAMES, frames), replace=False))
+    k = kps[pick].cpu().numpy()
+    fields = np.concatenate([k[..., :20].copy().view(np.float32), k[..., 20:].copy().view(np.int32).astype(np.float32)], axis=-1)
+    live = np.arange(cap)[None, :] < n[pick][:, None]
+    has_next = (pick < frames - 1)[:, None]
+    out = {"keypoint_count": n.astype(np.float64),
+           "match_count": np.where(np.arange(frames) < frames - 1, nmatch.cpu().numpy(), 0).astype(np.float64),
+           "sample_frames": pick.astype(np.float64),
+           "keypoints": np.where(live[..., None], fields, 0).astype(np.float32),
+           "descriptors": np.where(live[..., None], desc[pick].cpu().numpy(), 0).astype(np.float32),
+           "matches": np.where(live & has_next, match[pick].cpu().numpy(), -1).astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     from cubemapslam_b200.frontend import FrontEnd
@@ -182,6 +208,8 @@ def run_ours(args):
     ms_total = e0.elapsed_time(e1)
     launches = fe.launches + mt.launches - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, kps, desc, nout, match, nmatch)
     tms = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
@@ -483,7 +511,10 @@ def main():
     ap.add_argument("--pose-frames", type=int, default=2048)
     ap.add_argument("--track-frames", type=int, default=1024)
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

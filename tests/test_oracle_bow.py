@@ -1,23 +1,21 @@
-"""oracle DBoW2 transform (oracle/bow.h) == the reference's own DBoW2 compiled in oracle/_ref/libref.so, on a synthetic vocabulary in ORBvoc.txt's format."""
-import os
-
+"""oracle DBoW2 transform (oracle/bow.h) == the reference's own DBoW2 compiled in oracle/_ref/libref.so, on a synthetic vocabulary in ORBvoc.txt's format.
+The reference's results are read from tests/golden/ref_oracle_bow.npz (tests/refgold.py)."""
 import numpy as np
 import pytest
 
 from cubemapslam_b200 import synth
-
-ref = pytest.importorskip("oracle.ref")
-if not (ref.available() or os.path.isdir("/root/reference")):
-    pytest.skip("oracle/_ref/libref.so not built and no reference tree to build it from", allow_module_level=True)
+from oracle import ref
+from tests.refgold import RECORD, gold  # noqa: F401
 
 
 @pytest.mark.parametrize("k,L,levelsup", [(10, 4, 2), (6, 5, 4), (10, 3, 4)])
-def test_transform_matches_reference_dbow2(oracle, tmp_path, k, L, levelsup):
+def test_transform_matches_reference_dbow2(oracle, tmp_path, gold, k, L, levelsup):
     voc = synth.vocabulary(k=k, L=L, seed=k + L)
     path = tmp_path / "voc.txt"
     synth.write_vocabulary_text(voc, str(path))
-    rv = ref.RefVocabulary(str(path))
-    assert rv.size() == k ** L
+    rv = ref.RefVocabulary(str(path)) if RECORD else None
+    key = "k%d_L%d_up%d" % (k, L, levelsup)
+    assert gold.value("size_" + key, lambda: rv.size()) == k ** L
     ov = oracle.Vocabulary(k, L, voc["parent"], voc["is_leaf"], voc["desc"], voc["weight"])
     rng = np.random.default_rng(1)
     # features near words (realistic) plus pure noise
@@ -25,8 +23,7 @@ def test_transform_matches_reference_dbow2(oracle, tmp_path, k, L, levelsup):
     f1 = voc["desc"][rng.choice(leaves, 1500)] ^ np.packbits(rng.random((1500, 256)) < 0.05, axis=1, bitorder="little")
     feats = np.concatenate([f1, rng.integers(0, 256, (500, 32), dtype=np.uint8)])
     bw, bv, node, word = ov.transform(feats, levelsup)
-    rbw, rbv, rnode = rv.transform(feats, levelsup)
-    assert np.array_equal(bw, rbw) and np.array_equal(bv, rbv)            # BowVector: same words, bit-identical L1-normalised doubles
-    assert np.array_equal(node, rnode)                                    # FeatureVector membership of every feature
+    # BowVector: same words, bit-identical L1-normalised doubles; FeatureVector membership of every feature
+    assert gold.same("transform_" + key, (bw, bv, node), lambda: rv.transform(feats, levelsup))
     assert abs(bv.sum() - 1.0) < 1e-12 and len(bw) > 300
     assert (node[word >= 0] >= 0).mean() > 0.95                           # a few stopped words (weight 0) are excluded like in the reference
