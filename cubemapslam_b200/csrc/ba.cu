@@ -875,6 +875,40 @@ enum { NCCL_U8 = 1, NCCL_I32 = 2, NCCL_F64 = 8, NCCL_SUM = 0, NCCL_MAX = 2 };
 enum { BK_ERRORS = 0, BK_LIN_POINTS, BK_LIN_POSES, BK_DINV, BK_SCHUR, BK_XCHG, BK_SOLVE, BK_BACKSUB, BK_UPDATE, BK_SCALE, BK_END, BK_COUNT };
 static const char* kBaKindNames[BK_COUNT] = {"k_ba_errors", "k_ba_lin_points", "k_ba_lin_poses", "k_ba_dinv", "k_ba_schur", "exchange", "k_ba_solve", "k_ba_backsub", "k_ba_update", "k_ba_scale", "end"};
 
+// Dynamic shared memory of k_ba_solve: [staged panels 2 x NB x ldp] + y[n]. y alone caps the system at n = SOLVE_DSMEM / 8 = 26112 (4352 free key frames).
+static const int SOLVE_DSMEM = 204 * 1024;
+static const size_t SOLVE_STAGE_BYTES = 200 * 1024;   // the panels are staged when they and y fit in this
+
+// Shared-memory plan of k_ba_solve for an n x n system with panel stride ldp. stage: -1 = stage when it fits, 0 = panels read from L2, 1 = staged.
+static int solve_plan(int n, int ldp, int stage, int* stageOut, size_t* dsmem) {
+    const size_t panel = 2 * (size_t)LD_NB * ldp * 8, ybytes = (size_t)n * 8;
+    if (ybytes > (size_t)SOLVE_DSMEM) { set_error("reduced camera system n = %d exceeds the solver's shared-memory capacity (n <= %d, i.e. %d free key frames)", n, SOLVE_DSMEM / 8, SOLVE_DSMEM / 48); return CSLAM_E_CAPACITY; }
+    const bool fits = panel + ybytes <= SOLVE_STAGE_BYTES;
+    if (stage == 1 && !fits) { set_error("solve: staged panels do not fit in shared memory at n = %d", n); return CSLAM_E_BADARG; }
+    *stageOut = stage < 0 ? (fits ? 1 : 0) : stage;
+    *dsmem = (*stageOut ? panel : 0) + ybytes;
+    return 0;
+}
+
+static cudaLaunchConfig_t solve_config(cudaLaunchAttribute* at, int cluster, size_t dsmem, cudaStream_t s) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(cluster); cfg.blockDim = dim3(SOLVE_T); cfg.dynamicSmemBytes = dsmem; cfg.stream = s;
+    at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    return cfg;
+}
+
+// The one launch of k_ba_solve (LM trials and cslam_ba_solve_dense): one cluster of `cluster` CTAs factors R.S / R.g in place, writes R.xp and
+// sets R.scal[3] = 1 on a zero / non-finite pivot.
+static int launch_solve(cslam_optimizer* o, const BADev& R, double* Lt, double* LDt, double* Minv, int ldp, int stage, int cluster, long long* prof) {
+    int stg = 0; size_t dsmem = 0;
+    if (int rc = solve_plan(R.n, ldp, stage, &stg, &dsmem)) return rc;
+    cudaLaunchAttribute at[1];
+    const cudaLaunchConfig_t cfg = solve_config(at, cluster, dsmem, o->stream);
+    CSLAM_CUDA(cudaLaunchKernelEx(&cfg, k_ba_solve, R, Lt, LDt, Minv, ldp, stg, prof)); o->launches++;
+    return 0;
+}
+
 
 extern "C" int cslam_optimizer_create(cslam_optimizer** out, int device) {
     if (!out) return CSLAM_E_BADARG;
@@ -888,7 +922,7 @@ extern "C" int cslam_optimizer_create(cslam_optimizer** out, int device) {
     }
     if (const char* e = getenv("CSLAM_SOLVE_CLUSTER")) o->clusterSize = std::max(1, std::min(atoi(e), 16));
     if (o->clusterSize > 8) cudaFuncSetAttribute(k_ba_solve, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    cudaFuncSetAttribute(k_ba_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, 204 * 1024);
+    cudaFuncSetAttribute(k_ba_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, SOLVE_DSMEM);
     if (const char* e = getenv("CSLAM_BA_GRAPH")) o->useGraphs = atoi(e) != 0;
     *out = o;
     return CSLAM_OK;
@@ -917,6 +951,42 @@ extern "C" int cslam_optimizer_set_timing(cslam_optimizer* o, int enable) {
 extern "C" int cslam_optimizer_get_timing(const cslam_optimizer* o, int kind, const char** name, double* ms, int64_t* count) {
     if (!o || kind < 0 || kind >= BK_END) return CSLAM_E_BADARG;
     *name = kBaKindNames[kind]; *ms = o->kindMs[kind]; *count = o->kindCount[kind];
+    return CSLAM_OK;
+}
+
+extern "C" int cslam_ba_solve_dense(cslam_optimizer* o, int n, const double* Sg, int stage, int cluster, double* x, int32_t* failed) {
+    if (!o || !Sg || !x || !failed || n < 1 || stage < -1 || stage > 1 || cluster < 0 || cluster > 16) { set_error("cslam_ba_solve_dense: bad argument"); return CSLAM_E_BADARG; }
+    const int C = cluster ? cluster : o->clusterSize;
+    const int ldp = ((n + 1 + 8) + 3) & ~3;   // as cslam_local_ba sizes it
+    int rc, stg = 0; size_t dsmem = 0;
+    if ((rc = solve_plan(n, ldp, stage, &stg, &dsmem))) return rc;   // before anything touches Sg
+    CSLAM_CUDA(cudaSetDevice(o->device));
+    if (C > 8) CSLAM_CUDA(cudaFuncSetAttribute(k_ba_solve, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    {
+        cudaLaunchAttribute at[1];
+        const cudaLaunchConfig_t cfg = solve_config(at, C, dsmem, o->stream);
+        int nc = 0;
+        const cudaError_t e = cudaOccupancyMaxActiveClusters(&nc, k_ba_solve, &cfg);
+        if (e != cudaSuccess || nc == 0) {
+            cudaGetLastError();
+            set_error("solve: a cluster of %d CTAs with %zu B of dynamic shared memory each cannot be scheduled on this device (%s)", C, dsmem, cudaGetErrorString(e));
+            return CSLAM_E_BADARG;
+        }
+    }
+    free_pool(o);
+    BADev R; std::memset(&R, 0, sizeof(R));
+    R.n = n;
+    double *Lt = nullptr, *LDt = nullptr, *Minv = nullptr;
+    if ((rc = dalloc(o, &R.S, (size_t)(n + 1) * n)) || (rc = dalloc(o, &R.xp, n)) || (rc = dalloc(o, &R.scal, 8, true)) || (rc = dalloc(o, &Lt, (size_t)LD_NB * ldp)) ||
+        (rc = dalloc(o, &LDt, (size_t)LD_NB * ldp)) || (rc = dalloc(o, &Minv, (size_t)(n / LD_NB + 1) * LD_NB * LD_NB))) return rc;
+    R.g = R.S + (size_t)n * n;
+    CSLAM_CUDA(cudaMemcpyAsync(R.S, Sg, (size_t)(n + 1) * n * sizeof(double), cudaMemcpyHostToDevice, o->stream));
+    if ((rc = launch_solve(o, R, Lt, LDt, Minv, ldp, stg, C, nullptr))) return rc;
+    CSLAM_CUDA(cudaMemcpyAsync(x, R.xp, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, o->stream));
+    CSLAM_CUDA(cudaMemcpyAsync(o->h_scal, R.scal + 3, sizeof(double), cudaMemcpyDeviceToHost, o->stream));
+    CSLAM_CUDA(cudaStreamSynchronize(o->stream));
+    *failed = o->h_scal[0] != 0.0;
+    free_pool(o);
     return CSLAM_OK;
 }
 
@@ -1163,14 +1233,7 @@ struct BAHost {
             }
             CSLAM_CUDA(cudaMemsetAsync(D.scal + 3, 0, sizeof(double), o->stream));
             tick(BK_SOLVE);
-            const size_t panel = 2 * (size_t)LD_NB * ldp * 8, ybytes = (size_t)D.n * 8;
-            const int stage = panel + ybytes <= 200 * 1024 ? 1 : 0;
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(o->clusterSize); cfg.blockDim = dim3(SOLVE_T); cfg.dynamicSmemBytes = (stage ? panel : 0) + ybytes; cfg.stream = o->stream;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = o->clusterSize; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-            cfg.attrs = at; cfg.numAttrs = 1;
-            CSLAM_CUDA(cudaLaunchKernelEx(&cfg, k_ba_solve, R, Lt, LDt, Minv, ldp, stage, d_prof)); o->launches++;
+            if ((rc = launch_solve(o, R, Lt, LDt, Minv, ldp, -1, o->clusterSize, d_prof))) return rc;
         }
         tick(BK_BACKSUB);
         k_ba_backsub<<<grid(D.nMP * LM_LANES, 128), 128, 0, o->stream>>>(D); o->launches++;

@@ -42,6 +42,17 @@ class Optimizer:
                 out[name.value.decode()] = (ms.value, cnt.value)
         return out
 
+    def solve_dense(self, Sg, stage=-1, cluster=0):
+        """The reduced-camera-system solve of LocalBundleAdjustment on its own (test / measurement hook): Sg is (n+1) x n float64, S with the
+        right-hand side as row n; only the lower triangle of S is read. Returns (x, failed)."""
+        Sg = np.ascontiguousarray(Sg, np.float64)
+        n = Sg.shape[1]
+        if Sg.shape != (n + 1, n):
+            raise ValueError("Sg must be (n+1) x n, got %s" % (Sg.shape,))
+        x = np.empty(n); failed = C.c_int32()
+        check(lib().cslam_ba_solve_dense(self._h, int(n), ptr(Sg), int(stage), int(cluster), ptr(x), C.byref(failed)))
+        return x, bool(failed.value)
+
     @staticmethod
     def nccl_unique_id():
         buf = np.zeros(128, np.uint8)

@@ -244,6 +244,13 @@ int64_t cslam_optimizer_launches(const cslam_optimizer* o);
  * kind 0..9 = k_ba_errors, k_ba_lin_points, k_ba_lin_poses, k_ba_dinv, k_ba_schur, exchange, k_ba_solve, k_ba_backsub, k_ba_update, k_ba_scale. */
 int cslam_optimizer_set_timing(cslam_optimizer* o, int enable);
 int cslam_optimizer_get_timing(const cslam_optimizer* o, int kind, const char** name, double* ms, int64_t* count);
+/* Test / measurement hook (like cslam_ubench_*): the reduced-camera-system solve of cslam_local_ba alone, with the same launch, on a dense n x n
+ * symmetric system. Sg: host, (n+1) x n row-major, rows 0..n-1 = S (only the lower triangle is read), row n = the right-hand side g.
+ * stage: -1 = the production rule, 0 = trailing update reads the panels from L2, 1 = panels staged in shared memory (CSLAM_E_BADARG if they do
+ * not fit). cluster: CTAs of the solver cluster, 0 = the optimizer's own (CSLAM_SOLVE_CLUSTER, default 8), else 1..16 (> 8 is non-portable;
+ * CSLAM_E_BADARG if the device cannot schedule it). x: n doubles out, undefined when *failed. failed: 1 on a zero / non-finite pivot.
+ * n > 26112 (4352 free key frames) is CSLAM_E_CAPACITY, reported before Sg is read. */
+int cslam_ba_solve_dense(cslam_optimizer* o, int n, const double* Sg, int stage, int cluster, double* x, int32_t* failed);
 /* Landmark-sharded multi-GPU BA: every rank calls with the SAME problem; rank r owns landmarks l % nranks == r and
  * all-reduces the reduced camera system over NCCL. id128: ncclUniqueId bytes from cslam_nccl_unique_id on rank 0. */
 int cslam_nccl_unique_id(uint8_t id128[128]);

@@ -277,6 +277,8 @@ int orc_pose_opt(int n, float* Tcw, const float* Xw, const float* kpxy, const fl
     return inl;
 }
 // exposed pieces for unit tests
+// the reduced-camera-system solve of orc_local_ba: LDL^T without pivoting of the n x n row-major A (lower triangle read). 0 = zero / non-finite pivot.
+int orc_ldlt_solve(const double* A, int n, const double* b, double* x) { return ldlt_solve(std::vector<double>(A, A + (size_t)n * n), n, b, x, false) ? 1 : 0; }
 void orc_se3_exp(const double* u, double* out7) { SE3 s = se3_exp(u); out7[0] = s.t[0]; out7[1] = s.t[1]; out7[2] = s.t[2]; out7[3] = s.r.x; out7[4] = s.r.y; out7[5] = s.r.z; out7[6] = s.r.w; }
 void orc_edge_eval(const float* Tcw, const double* X, float kx, float ky, int faceW, int faceH, double* err2, double* Jp12, double* Jx6, int* face) {
     SE3 T = se3_from_Tcw32(Tcw); EdgeObs o = make_obs(kx, ky, 1.f, faceW, faceH); double Xc[3], R[3][3], Jp[2][6], Jx[2][3];

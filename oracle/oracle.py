@@ -381,6 +381,16 @@ def pose_opt(Tcw, Xw, kpxy, inv_sigma2, faceW, faceH):
     return dict(inliers=inl, Tcw=Tcw.reshape(4, 4), outlier=outlier[:n], pose64=pose64, log=log[:nit.value])
 
 
+def ldlt_solve(S, g):
+    """The dense LDL^T (no pivoting) local_ba solves its reduced camera system with; only the lower triangle of S is read.
+    Returns (x, ok); ok is False on a zero / non-finite pivot."""
+    S = np.ascontiguousarray(S, np.float64); g = np.ascontiguousarray(g, np.float64); n = len(g)
+    assert S.shape == (n, n)
+    x = np.zeros(n)
+    ok = lib().orc_ldlt_solve(_p(S), n, _p(g), _p(x))
+    return x, bool(ok)
+
+
 def se3_exp(u):
     u = np.ascontiguousarray(u, np.float64); out = np.zeros(7)
     lib().orc_se3_exp(_p(u), _p(out))
