@@ -86,6 +86,8 @@ class Optimizer:
         check(lib().cslam_optimizer_sync(self._h))
 
     def pose_optimization_dev(self, nframes, stride, count, Tcw, Xw, kpxy, inv_sigma2, faceW, faceH, outlier, inliers):
+        """Device addresses, asynchronous on self.stream; Tcw is updated in place. Outlier flags come back in the order of the correspondences
+        (after Tracker.gather_pose_inputs_dev: gathered order, not key-point slots)."""
         check(lib().cslam_pose_optimization_dev(self._h, int(nframes), int(stride), ptr(count), ptr(Tcw), ptr(Xw), ptr(kpxy), ptr(inv_sigma2), int(faceW), int(faceH), ptr(outlier),
                                                 ptr(inliers)))
 

@@ -265,8 +265,10 @@ int cslam_pose_optimization(cslam_optimizer* o, int nframes, const int32_t* offs
                             const float* kp_xy, const float* inv_sigma2, int face_w, int face_h, uint8_t* outlier,
                             int32_t* inliers, double* pose_fp64);
 
-/* Device-resident PoseOptimization for pipelines: frame f owns correspondences [f*stride, f*stride + count[f]); all pointers on the device;
- * asynchronous on the optimizer's stream (cslam_optimizer_stream / cslam_optimizer_sync). */
+/* Device-resident PoseOptimization for pipelines: frame f owns correspondences [f*stride, f*stride + min(count[f], stride)); all pointers on the device;
+ * asynchronous on the optimizer's stream (cslam_optimizer_stream / cslam_optimizer_sync). A frame with fewer than 3 correspondences keeps its Tcw
+ * and gets inliers 0. outlier[f*stride + i] belongs to correspondence i: after cslam_tracker_gather_pose_inputs_dev that is the gathered
+ * (compacted) order, and mapping the flags back to key-point slots is the caller's job. Bytes past the count are not written. */
 int cslam_pose_optimization_dev(cslam_optimizer* o, int nframes, int stride, const int32_t* count, float* Tcw, const float* Xw, const float* kp_xy, const float* inv_sigma2,
                                 int face_w, int face_h, uint8_t* outlier, int32_t* inliers);
 void* cslam_optimizer_stream(const cslam_optimizer* o);
